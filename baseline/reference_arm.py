@@ -1,7 +1,7 @@
 """Reference arm of bench.py: the UNMODIFIED reference (facebookresearch/mbrl-lib) on the host CPUs.
 
-``baseline/_ref`` holds ``pip install --no-deps --target baseline/_ref /root/reference`` (git-ignored, travels to the
-GPU box with the snapshot); in the build container ``/root/reference`` works too.  mbrl-lib imports hydra, omegaconf,
+The package is imported from ``oracle/_ref`` (the copy ``build()`` makes with ``oracle/ref_install.py``) or from
+``baseline/_ref`` (a ``pip install --no-deps --target`` of mbrl-lib); both are git-ignored.  mbrl-lib imports hydra, omegaconf,
 gymnasium and termcolor at module level; none of them is installed in this image and there is no index, so the
 API shims under ``oracle/ref_shims`` (a dict-backed DictConfig, ``hydra.utils.instantiate``, ``gymnasium.spaces.Box``)
 stand in for them.  They are configuration plumbing only: every tensor operation on the timed path
@@ -34,7 +34,7 @@ def import_reference():
         except ImportError:
             if shims not in sys.path:
                 sys.path.insert(0, shims)
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
+    for cand in (os.path.join(ROOT, "oracle", "_ref"), os.path.join(ROOT, "baseline", "_ref")):
         if os.path.isdir(os.path.join(cand, "mbrl")):
             sys.path.insert(0, cand)
             try:
@@ -51,7 +51,7 @@ def import_reference():
                     del sys.modules[k]
                 last = f"{cand}: {type(e).__name__}: {e}"
                 continue
-    return None, locals().get("last", "no baseline/_ref and no /root/reference")
+    return None, locals().get("last", "no oracle/_ref and no baseline/_ref")
 
 
 def _proc_fn(name):

@@ -6,7 +6,12 @@ population 500 candidate sequences, each rolled out for H = 30 steps with 20 par
 (7 members, 5 elites, 4 x 200 SiLU).  ``value`` times it device-resident (inputs in HBM, CUDA events);
 ``e2e`` times the public API call ``agent.act(obs)`` with a host observation in and the host plan out.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+``--dump-outputs DIR``: after the timed steps, the plan the last timed step returned (``CEMOptimizer.optimize``'s
+[H, A] solution, what ``agent.act`` hands back) is written to ``DIR/solution.npy`` (float32).  Every input is seeded
+(model weights, observation, the optimiser's and the model's random streams), so two runs with the same arguments
+plan from identical inputs and two builds can be compared output for output.
 
 N > 1 (under torchrun): weak scaling -- every rank plans over its own 500-sequence shard of a 500 x N
 population, ONE all-gather of local top-k records per CEM iteration (mbrl_lib_b200.dist); ``e2e`` is then
@@ -14,7 +19,7 @@ population, ONE all-gather of local top-k records per CEM iteration (mbrl_lib_b2
 The same run also reports BASELINE config 5 (fixed global populations 8 000 ... 64 000 sharded over the N GPUs,
 strong scaling) with the collective's share of an iteration, in ``config5_population_scan_sharded``.
 
-``--impl reference``: the UNMODIFIED reference (mbrl-lib from ``baseline/_ref``) timed on the host CPUs through
+``--impl reference``: the UNMODIFIED reference (mbrl-lib from ``oracle/_ref``) timed on the host CPUs through
 its own ``TrajectoryOptimizerAgent.act`` (rank 0 only); the oracle port is the fallback when it cannot be imported.
 """
 import argparse
@@ -318,6 +323,9 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
     device = f"cuda:{local}"
+    # the optimisers seed their sampling streams with torch.initial_seed(), which torch draws afresh in every process:
+    # pin it so that a run's plans depend on its arguments only
+    torch.manual_seed(0)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device(device))
     spec, arrays, env = build_problem(device)
@@ -372,10 +380,13 @@ def run_ours(args):
     for s, e in evs:
         flush.fill_(1)
         s.record()
-        step()
+        out = step()
         e.record()
     barrier()
     step_ms = [s.elapsed_time(e) for s, e in evs]
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "solution.npy"), out.float().cpu().numpy())
     total_ms = torch.tensor([sum(step_ms)], device=device, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
@@ -652,7 +663,13 @@ if __name__ == "__main__":
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--no-scan5", action="store_true", help="skip the sharded config-5 population scan (N > 1)")
     ap.add_argument("--no-scan", action="store_true", help="skip the population scan / extra configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's plan to DIR/solution.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the plan of the CUDA path; the reference arm draws its own random streams, "
+                 "so its outputs are not comparable output for output")
     if a.impl == "reference":
         run_reference(a)
     else:

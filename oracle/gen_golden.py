@@ -301,6 +301,50 @@ def gen_counter_world():
     print("counter_world", grid[8, 8].tolist())
 
 
+REFERENCE_OBJECT_CASES = ["halfcheetah_small", "cartpole", "hopper_tsinf", "pets_halfcheetah_small", "ant_learned_fn"]
+
+
+def gen_reference_objects():
+    """What tests/test_reference_objects.py checks the duck-typed boundary against: the recorded surface
+    (oracle/ref_surface.py) of the reference's OneDTransitionRewardModel(GaussianMLP) per case, of its reward /
+    termination callables, the shipped conf/action_optimizer/*.yaml and the optimizers' constructor arguments."""
+    import inspect
+    import json
+
+    import yaml
+
+    from oracle import ref_surface
+
+    models = {}
+    for name in REFERENCE_OBJECT_CASES:
+        spec = syn.CASES[name]
+        models[name] = ref_surface.record(build_reference(spec, syn.make_model_arrays(spec)).dynamics_model)
+    # the drop-in object of tests/test_host_cpu.py: fp64 normaliser, reward from reward_fns, no learned rewards
+    mlp = mbrl.models.GaussianMLP(23, 17, "cpu", num_layers=4, ensemble_size=7, hid_size=200,
+                                  propagation_method="random_model", activation_fn_cfg={"_target_": "torch.nn.SiLU"})
+    wrapper = mbrl.models.OneDTransitionRewardModel(mlp, target_is_delta=True, normalize=True,
+                                                    normalize_double_precision=True, learned_rewards=False, num_elites=5)
+    wrapper.set_elite([0, 2, 3, 5, 6])
+    models["silu_fp64_normalizer"] = ref_surface.record(wrapper)
+    conf = os.path.join(os.path.dirname(mbrl.__file__), "examples", "conf", "action_optimizer")
+    yamls = {}
+    for name in ("cem", "icem", "mppi"):
+        with open(os.path.join(conf, f"{name}.yaml")) as f:
+            yamls[name] = yaml.safe_load(f)
+    ctor = {c: sorted(set(inspect.signature(getattr(mbrl.planning, c).__init__).parameters) - {"self"})
+            for c in ("CEMOptimizer", "ICEMOptimizer", "MPPIOptimizer")}
+    out = {"models": models,
+           "reward_fns": {n: ref_surface.record(getattr(ref_rew, n))
+                          for n in ("cartpole", "cartpole_pets", "inverted_pendulum", "halfcheetah", "pusher")},
+           "termination_fns": {n: ref_surface.record(getattr(ref_term, n)) for n in
+                               ("hopper", "cartpole", "inverted_pendulum", "no_termination", "walker2d", "ant", "humanoid")},
+           "optimizer_yaml": yamls, "optimizer_ctor_args": ctor}
+    with open(os.path.join(GOLD, "reference_objects.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("reference_objects", sorted(models))
+
+
 if __name__ == "__main__":
     torch.manual_seed(0)
     os.makedirs(GOLD, exist_ok=True)
@@ -316,3 +360,4 @@ if __name__ == "__main__":
     gen_mppi()
     gen_cem_model()
     gen_counter_world()
+    gen_reference_objects()

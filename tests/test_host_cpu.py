@@ -122,31 +122,26 @@ def test_staging_signature_tracks_training_side_changes():
     assert len({s0, s1, s2, s3}) == 4
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/mbrl"), reason="reference tree only exists in the build container")
 def test_staging_reads_the_real_reference_objects():
-    """Drop-in check against mbrl-lib's own classes (imported with the API shims): the staging code must find every
-    attribute it needs on OneDTransitionRewardModel(GaussianMLP) and resolve mbrl's own reward / termination fns."""
-    import sys
+    """Drop-in check against mbrl-lib's own classes, as recorded from the imported reference (oracle/gen_golden.py,
+    oracle/ref_surface.py): the staging code must find every attribute it needs on OneDTransitionRewardModel(GaussianMLP)
+    -- GaussianMLP(23, 17, SiLU, 4 x 200, ensemble 7), fp64 normaliser, set_elite([0, 2, 3, 5, 6]) -- and resolve
+    mbrl's own reward / termination fns."""
+    import json
 
-    sys.path[:0] = [os.path.join(ROOT, "oracle", "ref_shims"), "/root/reference"]
-    try:
-        import mbrl.env.reward_fns as R
-        import mbrl.env.termination_fns as T
-        import mbrl.models
-    finally:
-        del sys.path[:2]
     from mbrl_lib_b200 import _lib, functions
     from mbrl_lib_b200.staging import StagedModel
+    from oracle import ref_surface
 
-    mlp = mbrl.models.GaussianMLP(23, 17, "cpu", num_layers=4, ensemble_size=7, hid_size=200,
-                                  propagation_method="random_model", activation_fn_cfg={"_target_": "torch.nn.SiLU"})
-    wrapper = mbrl.models.OneDTransitionRewardModel(mlp, target_is_delta=True, normalize=True,
-                                                    normalize_double_precision=True, learned_rewards=False, num_elites=5)
-    wrapper.set_elite([0, 2, 3, 5, 6])
+    with open(os.path.join(ROOT, "tests", "golden", "reference_objects.json")) as f:
+        rec = json.load(f)
+    R = {k: ref_surface.rebuild(v) for k, v in rec["reward_fns"].items()}
+    T = {k: ref_surface.rebuild(v) for k, v in rec["termination_fns"].items()}
+    wrapper = ref_surface.rebuild(rec["models"]["silu_fp64_normalizer"])
     st = StagedModel.__new__(StagedModel)
     st.src, st.mlp = wrapper, wrapper.model
-    st.reward_id = functions.resolve_reward(R.halfcheetah)
-    st.term_id = functions.resolve_term(T.no_termination)
+    st.reward_id = functions.resolve_reward(R["halfcheetah"])
+    st.term_id = functions.resolve_term(T["no_termination"])
     d = st._describe()
     assert (d.ensemble_size, d.num_members, d.obs_dim, d.act_dim, d.in_size, d.out_size, d.hid_size, d.num_hidden) == \
         (7, 5, 17, 6, 23, 17, 200, 4)
@@ -155,9 +150,9 @@ def test_staging_reads_the_real_reference_objects():
     assert st.members() == [0, 2, 3, 5, 6]
     assert [tuple(l.weight.shape) for l in st._layers()] == [(7, 23, 200)] + [(7, 200, 200)] * 3 + [(7, 200, 34)]
     for name in ("cartpole", "cartpole_pets", "inverted_pendulum", "pusher"):
-        assert functions.resolve_reward(getattr(R, name)) == _lib.REWARD[name]
+        assert functions.resolve_reward(R[name]) == _lib.REWARD[name]
     for name in ("hopper", "cartpole", "inverted_pendulum", "walker2d", "ant", "humanoid"):
-        assert functions.resolve_term(getattr(T, name)) == _lib.TERM[name]
+        assert functions.resolve_term(T[name]) == _lib.TERM[name]
 
 
 def test_rollout_model_env_protocol():

@@ -1,16 +1,22 @@
 """The drop-in boundary against REAL mbrl-lib objects (SURVEY.md 8b; VERDICT r1 "boundary is a mirror, never a plug-in").
 
-The unmodified reference is imported from ``baseline/_ref`` (the pip --target install that travels to the GPU box) or
-``/root/reference`` (build container), with the four absent pure-Python deps shimmed (``oracle/ref_shims``).
+``tests/golden/reference_objects.json`` holds what ``oracle/gen_golden.py`` recorded from the unmodified reference
+(imported with the four absent pure-Python deps shimmed, ``oracle/ref_shims``): the attribute surface of its
+``OneDTransitionRewardModel(GaussianMLP)`` objects, its reward / termination callables, the shipped
+``conf/action_optimizer/{cem,icem,mppi}.yaml`` and the optimizers' constructor arguments.  ``oracle.ref_surface.rebuild``
+turns a recorded model back into an object with exactly the recorded attributes, so the checks below read what
+the real object exposes without mbrl-lib being installed:
 
-* CPU (here): ``staging.StagedModel(stage=False)`` reads a real ``mbrl.models.OneDTransitionRewardModel(GaussianMLP)``
-  after ``set_elite`` / ``update_normalizer`` exactly as the kernels need it, its signature notices what
-  ``ModelTrainer`` / ``Normalizer.update_stats`` change between ``act()`` calls, the reference's own reward /
-  termination callables resolve to device functions, and the shipped ``conf/action_optimizer/{cem,icem,mppi}.yaml``
-  instantiate through ``_instantiate`` into the B200 classes.
-* GPU: the real reference model object lives on cuda:0; OUR ``ModelEnv`` wraps it and must reproduce what the
-  REFERENCE's ``ModelEnv.evaluate_action_sequences`` computes on the very same object with the same injected draws.
+* CPU: ``staging.StagedModel(stage=False)`` reads the recorded objects exactly as the kernels need them, the
+  reference's own reward / termination callables resolve to device functions, and the shipped YAMLs instantiate
+  through ``_instantiate`` into the B200 classes.
+* GPU: OUR ``ModelEnv`` over the recorded reference object (weights filled in) must reproduce what the REFERENCE's
+  ``ModelEnv.evaluate_action_sequences`` computed with the same injected draws (``tests/golden/rollout_<case>.npz``).
+
+Three tests exercise mbrl-lib's own code (its trainer, normaliser and class hierarchy).  They import the unmodified
+package that ``build()`` copies into ``oracle/_ref`` (``oracle/ref_install.py``) and skip where no copy could be made.
 """
+import json
 import os
 import sys
 
@@ -23,9 +29,42 @@ sys.path.insert(0, ROOT)
 
 from baseline import reference_arm as ra  # noqa: E402
 from mbrl_lib_b200 import _lib, functions, staging, synthetic as syn  # noqa: E402
+from oracle import ref_surface  # noqa: E402
 
 mbrl, REF_SRC = ra.import_reference()
-needs_ref = pytest.mark.skipif(mbrl is None, reason=f"reference not importable here: {REF_SRC}")
+needs_ref = pytest.mark.skipif(mbrl is None, reason=f"mbrl-lib not importable here: {REF_SRC}")
+with open(os.path.join(ROOT, "tests", "golden", "reference_objects.json")) as _f:
+    RECORDED = json.load(_f)
+
+
+def _recorded_model(name, device="cpu"):
+    """The reference's OneDTransitionRewardModel(GaussianMLP) of case ``name`` as recorded, carrying the synthetic
+    weights of the case (what oracle/gen_golden.py:build_reference loads into the real object)."""
+    spec = syn.CASES[name]
+    arrays = syn.make_model_arrays(spec)
+    wrapper = ref_surface.rebuild(RECORDED["models"][name], device)
+    mlp = wrapper.model
+    for li, layer in enumerate(mlp.hidden_layers):
+        layer[0].weight.copy_(torch.from_numpy(arrays["weights"][li]))
+        layer[0].bias.copy_(torch.from_numpy(arrays["biases"][li]))
+    mlp.mean_and_logvar.weight.copy_(torch.from_numpy(arrays["weights"][-1]))
+    mlp.mean_and_logvar.bias.copy_(torch.from_numpy(arrays["biases"][-1]))
+    if not spec.deterministic:
+        mlp.min_logvar.copy_(torch.from_numpy(arrays["min_logvar"]))
+        mlp.max_logvar.copy_(torch.from_numpy(arrays["max_logvar"]))
+    if spec.normalize is not None:
+        wrapper.input_normalizer.mean = torch.from_numpy(arrays["norm_mean"]).to(device)
+        wrapper.input_normalizer.std = torch.from_numpy(arrays["norm_std"]).to(device)
+    fn = wrapper.obs_process_fn
+    if fn is not None:  # the reference's Env.preprocess_fn was restated as a lambda (the env modules need mujoco): tag it
+        fn.b200pets_kind, fn.b200pets_name = "proc", spec.obs_process
+    return spec, arrays, wrapper
+
+
+def _recorded_callables(spec):
+    """The reference's own reward_fns.<name> / termination_fns.<name> of the case (recorded module and name)."""
+    rew = ref_surface.rebuild(RECORDED["reward_fns"][spec.reward_fn]) if spec.reward_fn else None
+    return rew, ref_surface.rebuild(RECORDED["termination_fns"][spec.term_fn])
 
 
 def _real_model(name="halfcheetah_small", device="cpu"):
@@ -47,12 +86,12 @@ def _real_model(name="halfcheetah_small", device="cpu"):
     return spec, arrays, env
 
 
-@needs_ref
 def test_staging_reads_a_real_reference_model():
-    spec, arrays, env = _real_model("halfcheetah_small")
-    wrapper = env.dynamics_model
-    assert type(wrapper).__module__.startswith("mbrl.models") and type(wrapper.model).__name__ == "GaussianMLP"
-    sm = staging.StagedModel(wrapper, env.reward_fn, env.termination_fn, stage=False)
+    rec = RECORDED["models"]["halfcheetah_small"]  # recorded from mbrl-lib's own classes
+    assert rec["class_module"].startswith("mbrl.models") and rec["attrs"]["model"]["class_module"].startswith("mbrl.models")
+    assert (rec["class"], rec["attrs"]["model"]["class"]) == ("OneDTransitionRewardModel", "GaussianMLP")
+    spec, arrays, wrapper = _recorded_model("halfcheetah_small")
+    sm = staging.StagedModel(wrapper, *_recorded_callables(spec), stage=False)
     d = sm._describe()
     assert (d.ensemble_size, d.num_members) == (spec.ensemble_size, spec.num_models)
     assert (d.in_size, d.out_size, d.hid_size, d.num_hidden) == (spec.in_size, spec.out_size, spec.hid_size, spec.num_layers)
@@ -105,38 +144,23 @@ def test_signature_follows_training_side_mutations():
     assert sm._signature() != s3 and sm._describe().norm_mode == 2
 
 
-@needs_ref
 def test_reference_callables_resolve_to_device_functions():
-    import mbrl.env.reward_fns as rr
-    import mbrl.env.termination_fns as rt
-
+    rr, rt = RECORDED["reward_fns"], RECORDED["termination_fns"]
     for name in ("cartpole", "cartpole_pets", "inverted_pendulum", "halfcheetah", "pusher"):
-        assert functions.resolve_reward(getattr(rr, name)) == _lib.REWARD[name]
+        assert functions.resolve_reward(ref_surface.rebuild(rr[name])) == _lib.REWARD[name]
     for name in ("hopper", "cartpole", "inverted_pendulum", "no_termination", "walker2d", "ant", "humanoid"):
-        assert functions.resolve_term(getattr(rt, name)) == _lib.TERM[name]
+        assert functions.resolve_term(ref_surface.rebuild(rt[name])) == _lib.TERM[name]
     assert functions.resolve_reward(None) == _lib.REWARD["learned"]
     assert functions.resolve_reward(lambda a, o: o[:, :1]) == _lib.REWARD["external"]
 
 
-def _shipped_yaml(rel):
-    import yaml
-
-    for base in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        path = os.path.join(base, "mbrl", "examples", "conf", "action_optimizer", rel)
-        if os.path.exists(path):
-            with open(path) as f:
-                return yaml.safe_load(f)
-    pytest.skip("shipped YAMLs not found")
-
-
-@needs_ref
 @pytest.mark.parametrize("name", ["cem", "icem", "mppi"])
 def test_shipped_optimizer_yaml_instantiates_into_b200_class(name, monkeypatch):
     """conf/action_optimizer/*.yaml carry `_target_: mbrl.planning.<X>Optimizer`, ${...} interpolations resolved here by
     hand (hydra does it in the reference, trajectory_opt.py:516-531 passes lower/upper bound itself)."""
     from mbrl_lib_b200 import planning
 
-    cfg = _shipped_yaml(f"{name}.yaml")
+    cfg = RECORDED["optimizer_yaml"][name]
     assert cfg["_target_"].startswith("mbrl.planning.")
     resolved = {}
     for k, v in cfg.items():
@@ -168,8 +192,7 @@ def test_shipped_optimizer_yaml_instantiates_into_b200_class(name, monkeypatch):
     real_cls = {"CEMOptimizer": planning.CEMOptimizer, "ICEMOptimizer": planning.ICEMOptimizer,
                 "MPPIOptimizer": planning.MPPIOptimizer}[expect]
     ours = set(inspect.signature(real_cls.__init__).parameters) - {"self"}
-    ref_cls = getattr(mbrl.planning, expect)
-    theirs = set(inspect.signature(ref_cls.__init__).parameters) - {"self"}
+    theirs = set(RECORDED["optimizer_ctor_args"][expect])
     assert set(captured["kw"]) <= ours, set(captured["kw"]) - ours
     assert theirs <= ours, f"reference ctor args missing from ours: {theirs - ours}"
 
@@ -219,27 +242,36 @@ class _Feed:
         torch.randperm, torch.normal = self._rp, self._nm
 
 
-@needs_ref
+class _Box:
+    def __init__(self, lo, hi, n):
+        self.low, self.high, self.shape = np.full(n, lo, np.float32), np.full(n, hi, np.float32), (n,)
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["halfcheetah_small", "cartpole", "hopper_tsinf", "pets_halfcheetah_small", "ant_learned_fn"])
 @pytest.mark.parametrize("precision,tol", [("f32", 2e-4), ("bf16_tc", 2e-2)])
-def test_our_model_env_on_real_reference_model_matches_reference_model_env(name, precision, tol):
+def test_our_model_env_on_real_reference_model_matches_reference_model_env(golden_dir, name, precision, tol):
     import mbrl_lib_b200 as bp
 
     dev = "cuda:0"
-    spec, arrays, ref_env = _real_model(name, dev)
+    spec, arrays, wrapper = _recorded_model(name, dev)
     inp = syn.make_rollout_inputs(spec)
+    # the reference's ModelEnv.evaluate_action_sequences on its own object with these draws (oracle/gen_golden.py)
+    gold = np.load(os.path.join(golden_dir, f"rollout_{name}.npz"))
+    assert str(gold["model_sum"]) == syn.checksum(arrays) and str(gold["input_sum"]) == syn.checksum(inp)
+    want = gold["returns"].astype(np.float32)
     acts = torch.from_numpy(inp["actions"]).to(dev)
     perms = torch.from_numpy(inp["perms"]).to(dev)
     eps = torch.from_numpy(inp["eps"]).to(dev)
-    H = spec.horizon
-    feed_perms = [] if spec.propagation == "expectation" else [perms[t] for t in range(perms.shape[0])]
-    feed_norm = [] if spec.deterministic else [eps[t] for t in range(H)]
-    with _Feed(feed_perms, feed_norm):
-        want = ref_env.evaluate_action_sequences(acts, inp["obs0"], spec.particles).float().cpu().numpy()
-    # ours, wrapping the SAME wrapper object and the reference's own reward / termination callables
-    env = bp.ModelEnv(ref_env, ref_env.dynamics_model, ref_env.termination_fn, ref_env.reward_fn,
-                      generator=torch.Generator(device=dev), precision=precision, ts1="perms")
+
+    class _Env:
+        observation_space = _Box(-np.inf, np.inf, spec.obs_dim)
+        action_space = _Box(spec.action_lb, spec.action_ub, spec.act_dim)
+
+    # ours, wrapping the reference's model object and its own reward / termination callables
+    reward_fn, term_fn = _recorded_callables(spec)
+    env = bp.ModelEnv(_Env(), wrapper, term_fn, reward_fn, generator=torch.Generator(device=dev), precision=precision,
+                      ts1="perms")
     if precision == "bf16_tc" and not env.staged.supports_tc():
         pytest.skip("dims outside the tensor-core plan")
     got = env.evaluate_action_sequences(acts, inp["obs0"], spec.particles, _perms=perms, _eps=eps).cpu().numpy()
