@@ -160,8 +160,11 @@ __global__ void particle_mean_kernel(int N, int P, const float* __restrict__ tot
 constexpr int kSelThreads = 1024;
 constexpr int kSmallN = 2048;  // populations up to this size are ranked by counting in shared memory
 
+// Order-preserving key of a float for the radix selects.  -0.0 maps to the key of +0.0: the two compare equal, so they
+// tie (lowest index first) exactly as in the counting paths and in torch.topk's comparisons.
 __device__ __forceinline__ uint32_t order_key(float v) {
   uint32_t u = __float_as_uint(v);
+  if (u == 0x80000000u) u = 0u;
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 

@@ -1,6 +1,6 @@
 """CPU oracle for the PETS planning hot path -- TEST INFRASTRUCTURE ONLY.
 
-This is a restatement (torch CPU ops, fp32, all randomness *injected*) of what the reference computes on
+This is a restatement (torch CPU ops, fp32 -- or fp64 on request --, all randomness *injected*) of what the reference computes on
 the path  CEMOptimizer/ICEMOptimizer -> ModelEnv.evaluate_action_sequences -> OneDTransitionRewardModel
 -> GaussianMLP.  It is the checker for the CUDA path; nothing in the product imports it.  Only
 ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s CPU-baseline / ``--impl reference`` legs may.
@@ -124,7 +124,8 @@ OBS_PROCESS: Dict[str, Callable] = {"halfcheetah": proc_halfcheetah, "cartpole":
 
 
 def _bf16_round(x: torch.Tensor) -> torch.Tensor:
-    return x.to(torch.bfloat16).to(torch.float32)
+    """round to bf16 and back to the working dtype (the products and sums stay in that dtype)."""
+    return x.to(torch.bfloat16).to(x.dtype)
 
 
 def _bf16_split_bias(b: torch.Tensor) -> torch.Tensor:
@@ -134,17 +135,31 @@ def _bf16_split_bias(b: torch.Tensor) -> torch.Tensor:
 
 
 class OracleModel:
-    """GaussianMLP ensemble wrapped as a OneDTransitionRewardModel, inference only."""
+    """GaussianMLP ensemble wrapped as a OneDTransitionRewardModel, inference only.
 
-    def __init__(self, spec, arrays):
+    ``dtype=torch.float64`` runs the whole path (model input, layers, sampling, delta targets, rewards, accumulation) in
+    double: the high-precision yardstick the kernels' error is measured against.  The float32 default is the reference's
+    own arithmetic, pinned bit-exact to the goldens."""
+
+    def __init__(self, spec, arrays, dtype=torch.float32):
         self.spec = spec
-        self.weights = [torch.from_numpy(np.asarray(w)) for w in arrays["weights"]]
-        self.biases = [torch.from_numpy(np.asarray(b)) for b in arrays["biases"]]
-        self.min_logvar = torch.from_numpy(np.asarray(arrays["min_logvar"]))
-        self.max_logvar = torch.from_numpy(np.asarray(arrays["max_logvar"]))
-        self.norm_mean = torch.from_numpy(arrays["norm_mean"]) if "norm_mean" in arrays else None
-        self.norm_std = torch.from_numpy(arrays["norm_std"]) if "norm_std" in arrays else None
-        self.members = list(spec.elites) if spec.elites is not None else list(range(spec.ensemble_size))
+        self.dtype = dtype
+        cast = lambda a: torch.from_numpy(np.asarray(a)).to(dtype)  # noqa: E731 (a no-op for the float32 arrays in fp32 mode)
+        self.weights = [cast(w) for w in arrays["weights"]]
+        self.biases = [cast(b) for b in arrays["biases"]]
+        self.min_logvar = cast(arrays["min_logvar"])
+        self.max_logvar = cast(arrays["max_logvar"])
+        # the normaliser keeps its own dtype in fp32 mode (an fp64 normaliser promotes, then .float(), as the reference)
+        self.norm_mean = self.norm_std = None
+        if "norm_mean" in arrays:
+            self.norm_mean = torch.from_numpy(arrays["norm_mean"])
+            self.norm_std = torch.from_numpy(arrays["norm_std"])
+            if dtype == torch.float64:
+                self.norm_mean, self.norm_std = self.norm_mean.double(), self.norm_std.double()
+        # gaussian_mlp.py:377-379: set_elite ignores a list that names as many members as the ensemble has (whatever its
+        # order): all members then run in index order
+        elites = spec.elites if spec.elites is not None and len(spec.elites) != spec.ensemble_size else None
+        self.members = list(elites) if elites is not None else list(range(spec.ensemble_size))
         self.emulate_bf16 = False
 
     # mbrl/models/gaussian_mlp.py:89-111 (activation choice), models/util.py:53-65 (layer)
@@ -185,7 +200,7 @@ class OracleModel:
             obs = OBS_PROCESS[self.spec.obs_process](obs)
         x = torch.cat([obs, act], dim=obs.ndim - 1)
         if self.norm_mean is not None:
-            x = ((x - self.norm_mean) / self.norm_std).float()
+            x = ((x - self.norm_mean) / self.norm_std).to(self.dtype)
         return x
 
     def forward_assigned(self, x: torch.Tensor, assign: torch.Tensor):
@@ -208,8 +223,8 @@ class OracleModel:
             finally:
                 self.members = keep
             if mean_out is None:
-                mean_out = torch.empty(B, mean.shape[-1])
-                lv_out = torch.empty(B, lv.shape[-1]) if lv is not None else None
+                mean_out = torch.empty(B, mean.shape[-1], dtype=mean.dtype)
+                lv_out = torch.empty(B, lv.shape[-1], dtype=lv.dtype) if lv is not None else None
             mean_out[rows] = mean[0]
             if lv is not None:
                 lv_out[rows] = lv[0]
@@ -242,6 +257,7 @@ class OracleModel:
         """ModelEnv.step (model_env.py:87-140) over OneDTransitionRewardModel.sample (one_dim_tr_model.py
         :245-289) and Ensemble.sample_1d (model.py:426-473).  Returns next_obs, reward[B,1], done[B,1]."""
         sp = self.spec
+        obs, act = obs.to(self.dtype), act.to(self.dtype)
         x = self.model_input(obs, act)
         mean, lv = self.forward_propagated(x, perm, assign)
         if sp.deterministic or not sample:
@@ -267,8 +283,8 @@ class OracleModel:
         N, H, _ = actions.shape
         P = particles
         B = N * P
-        obs = torch.from_numpy(np.tile(np.asarray(obs0), (B, 1)).astype(np.float32))
-        total = torch.zeros(B, 1)
+        obs = torch.from_numpy(np.tile(np.asarray(obs0), (B, 1)).astype(np.float32)).to(self.dtype)
+        total = torch.zeros(B, 1, dtype=self.dtype)
         dead = torch.zeros(B, 1, dtype=torch.bool)
         for t in range(H):
             a = torch.repeat_interleave(actions[:, t, :], P, dim=0)

@@ -32,6 +32,85 @@ def test_rollout_matches_reference(golden_dir, name):
     np.testing.assert_allclose(ret.numpy(), g["returns"], rtol=1e-6, atol=1e-6)
 
 
+@pytest.mark.parametrize("name", ROLLOUT_CASES)
+def test_float64_oracle_matches_reference(golden_dir, name):
+    """The double-precision oracle (the yardstick of tests/test_gpu_shapes.py) differs from the reference's fp32
+    arithmetic by rounding only: 1e-5 of the return scale on every golden rollout."""
+    spec = syn.CASES[name]
+    arrays = syn.make_model_arrays(spec)
+    inp = syn.make_rollout_inputs(spec)
+    g = _load(golden_dir, f"rollout_{name}.npz")
+    m = po.OracleModel(spec, arrays, dtype=torch.float64)
+    ret = m.evaluate_action_sequences(torch.from_numpy(inp["actions"]), inp["obs0"], spec.particles,
+                                      torch.from_numpy(inp["perms"]), torch.from_numpy(inp["eps"]))
+    assert ret.dtype == torch.float64
+    scale = max(1.0, float(np.abs(g["returns"]).max()))
+    err = float(np.abs(ret.numpy() - g["returns"]).max())
+    assert err <= 1e-5 * scale, f"max |diff| {err:.3e} > 1e-5 * {scale:.3g}"
+
+
+@pytest.mark.parametrize("name,batch", [("mbpo_halfcheetah_small", 1000), ("cartpole", 500)])
+def test_float64_oracle_step_matches_reference(golden_dir, name, batch):
+    spec = syn.CASES[name]
+    arrays = syn.make_model_arrays(spec)
+    inp = syn.make_step_inputs(spec, batch)
+    g = _load(golden_dir, f"step_{name}.npz")
+    m = po.OracleModel(spec, arrays, dtype=torch.float64)
+    nobs, rew, done = m.step(torch.from_numpy(inp["obs"]), torch.from_numpy(inp["act"]),
+                             torch.from_numpy(inp["perm"]), torch.from_numpy(inp["eps"]))
+    scale = max(1.0, float(np.abs(g["next_obs"]).max()))
+    assert np.abs(nobs.numpy() - g["next_obs"]).max() <= 1e-5 * scale
+    assert np.abs(rew.numpy() - g["reward"]).max() <= 1e-5 * scale
+    assert (done.numpy() == g["done"]).all()
+
+
+def test_float64_bf16_emulation_keeps_double_accumulation():
+    """emulate_bf16 in fp64 mode rounds the operands (activations, weights, the two bias parts) to bf16 and nothing
+    else: products and sums stay in double.  Restated layer by layer with numpy float64."""
+    x = torch.tensor([1.0 + 2.0 ** -7, 1.0 + 2.0 ** -9], dtype=torch.float64)
+    assert po._bf16_round(x).dtype == torch.float64
+    assert po._bf16_round(x).tolist() == [1.0 + 2.0 ** -7, 1.0]  # 8 significant bits, round to nearest even
+    spec = syn.CASES["tc_hid64"]
+    arrays = syn.make_model_arrays(spec)
+    m = po.OracleModel(spec, arrays, dtype=torch.float64)
+    m.emulate_bf16 = True
+    xs = torch.randn(len(m.members), 16, spec.in_size, generator=torch.Generator().manual_seed(0), dtype=torch.float64)
+    mean, lv = m.mlp(xs)
+    assert mean.dtype == torch.float64 and lv.dtype == torch.float64
+
+    def bf(a):
+        return torch.from_numpy(np.asarray(a, np.float64)).to(torch.bfloat16).double().numpy()
+
+    h = xs.numpy()
+    for li, (w, b) in enumerate(zip(arrays["weights"], arrays["biases"])):
+        w, b = w[m.members].astype(np.float64), b[m.members].astype(np.float64)
+        h = np.matmul(bf(h), bf(w)) + (bf(b) + bf(b - bf(b)))
+        if li < len(arrays["weights"]) - 1:
+            h = h / (1.0 + np.exp(-h))  # SiLU
+    np.testing.assert_allclose(mean.numpy(), h[..., :spec.out_size], rtol=1e-12, atol=1e-12)
+    m32 = po.OracleModel(spec, arrays)
+    m32.emulate_bf16 = True
+    mean32, _ = m32.mlp(xs.float())
+    assert not np.array_equal(mean32.double().numpy(), mean.numpy())  # fp32 accumulation rounds differently
+
+
+def test_full_elite_list_keeps_member_order():
+    """GaussianMLP.set_elite (gaussian_mlp.py:377-379) ignores an elite list as long as the ensemble: a reordered full
+    list runs the members in index order, exactly like no list."""
+    import dataclasses
+
+    base = dataclasses.replace(syn.CASES["tc_hid64"], elites=None)
+    arrays = syn.make_model_arrays(base)
+    inp = syn.make_rollout_inputs(base)
+    args = (torch.from_numpy(inp["actions"]), inp["obs0"], base.particles, torch.from_numpy(inp["perms"]),
+            torch.from_numpy(inp["eps"]))
+    ref = po.OracleModel(base, arrays).evaluate_action_sequences(*args)
+    full = po.OracleModel(dataclasses.replace(base, elites=(2, 0, 1)), arrays)
+    assert full.members == [0, 1, 2]
+    assert torch.equal(full.evaluate_action_sequences(*args), ref)
+    assert po.OracleModel(dataclasses.replace(base, elites=(2, 0)), arrays).members == [2, 0]  # a true subset keeps its order
+
+
 @pytest.mark.parametrize("name", ["halfcheetah_small", "hopper_tsinf", "ant_learned_fn", "tc_hid64"])
 def test_assigned_members_path_equals_permutation_path(name):
     """``forward_assigned`` (row -> member map given directly; what the GPU tile-shuffle tests feed the oracle) equals the
